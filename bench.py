@@ -80,11 +80,20 @@ def parse():
                         "the dibr_b200_peer_push kernel, nccl = all_gather_into_tensor; auto = peer when CUDA "
                         "symmetric memory can be set up on this box, else nccl")
     p.add_argument("--push-ctas", type=int, default=32, help="--gather peer_sm: grid of the push kernel")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step computed (features, soft_mask, "
+                        "face_idx, grad_face_vertices_image, grad_face_features) as DIR/<name>.npy in float32 / "
+                        "float64, at most 64 MB in all (a fixed seeded sample of the pixels / faces when larger). "
+                        "--impl ours only. With --gpus N, rank 0 writes: the images of its own views and the "
+                        "gradients as every rank receives them, all-gathered over the N x views")
     p.add_argument("--chunks", type=int, default=1,
                    help="N > 1: 1 = the all-gather of grad_face_features overlaps the soft-mask branch of "
                         "the backward (default); k > 1 = k view-chunks per step, chunk i's all-gather "
                         "overlaps chunk i+1 (measured slower at 32 views per GPU: smaller launches)")
-    return p.parse_args()
+    args = p.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs writes what the timed GPU step computed: --impl ours only")
+    return args
 
 
 def peaks():
@@ -339,10 +348,12 @@ def run_ours(args):
 
     def step_resident(ev=None):
         chunked = ChunkedGradAllGather(B) if world > 1 and len(spans) > 1 else None
+        images = []
         for ci, (c0, c1) in enumerate(spans):
             if ev: ev[3 * ci].record()
             feat, idx, wts, soft, ws = _host.forward(mode, H, W, d_fvz[c0:c1], d_fvi[c0:c1], d_ff[c0:c1],
                                                      d_fnz[c0:c1], None, MULT, EPS, SIGMAINV, boxlen_m, KNUM)
+            images.append((feat, soft, idx))
             if ev: ev[3 * ci + 1].record()
             bwd = lambda hook=None: _host.backward(H, W, g_feat[c0:c1], g_soft[c0:c1], idx, wts, soft,
                                                    d_fvi[c0:c1], d_ff[c0:c1], MULT, EPS, SIGMAINV, boxlen_m,
@@ -367,7 +378,7 @@ def run_ours(args):
                     chunked.submit(c0, c1, [g_fvi, g_ff])
         if chunked is not None:
             g_fvi, g_ff = chunked.finish()
-        return g_fvi, g_ff
+        return images, g_fvi, g_ff
 
     graph = None
     if args.graph and world == 1:
@@ -400,7 +411,9 @@ def run_ours(args):
     barrier()
     start.record()
     for k in range(args.steps):
-        step_resident(evs[k])
+        last = step_resident(evs[k])
+        if k + 1 < args.steps:
+            del last                    # each step's outputs are released before the next step, as in a loop
     end.record()
     barrier()
     clocks = sampler.stop() if sampler is not None else None
@@ -424,6 +437,9 @@ def run_ours(args):
     value = world * B * H * W / (ms_per_step * 1e-3) / 1e6
     step_stats = {"min": min(step_ms), "median": statistics.median(step_ms), "max": max(step_ms),
                   "rank": 0, "per_rank_mean_min_median_max": per_rank}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
 
     # ---- the backward scatter kernel alone (roofline kernel) ---------------
     feat, idx, wts, soft, ws = _host.forward(mode, H, W, d_fvz, d_fvi, d_ff, d_fnz, None, MULT, EPS,
@@ -753,6 +769,35 @@ def run_ours(args):
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BUDGET = 60 << 20     # bytes of all dumped arrays together (under 64 MB with the .npy headers)
+
+
+def dump_outputs(out_dir, last_step):
+    """Write what one resident step returned as <name>.npy: float32, face_idx as float64.  When the set
+    exceeds DUMP_BUDGET, the images share one seeded sample of pixels and the gradients one of faces
+    (rows of the flattened (B, H, W) / (B, F) leading dimensions, in increasing order), sized so that
+    the set fits.  The same arguments give the same inputs and the same rows, so two builds can be
+    compared output for output (the gradients accumulate with float atomics: compare them with a
+    tolerance, the images bit for bit)."""
+    import torch
+    images, g_fvi, g_ff = last_step
+    arrays = {"features": torch.cat([f for f, _, _ in images]), "soft_mask": torch.cat([s for _, s, _ in images]),
+              "face_idx": torch.cat([i for _, _, i in images]),
+              "grad_face_vertices_image": g_fvi, "grad_face_features": g_ff}
+    lead = {n: 3 if n in ("features", "soft_mask", "face_idx") else 2 for n in arrays}
+    rows = {n: t.shape[:lead[n]].numel() for n, t in arrays.items()}
+    nbytes = sum(t.numel() * (8 if t.dtype == torch.int64 else 4) for t in arrays.values())
+    keep = min(1.0, DUMP_BUDGET / max(nbytes, 1))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        out = t.detach().reshape(rows[name], -1)
+        if keep < 1.0:
+            sel = np.random.default_rng(lead[name]).choice(rows[name], int(rows[name] * keep), replace=False)
+            out = out[torch.from_numpy(np.sort(sel)).to(out.device)]
+        out = out.to(torch.float64 if t.dtype == torch.int64 else torch.float32).cpu().numpy()   # bf16 too
+        np.save(os.path.join(out_dir, name + ".npy"), out.reshape(t.shape) if keep >= 1.0 else out)
 
 
 def time_reference_cuda(args, dev, B, F, H, W, D, d_fvz, d_fvi, d_ff, d_fnz, g_feat, g_soft):

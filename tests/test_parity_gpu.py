@@ -5,8 +5,8 @@ forward floats within 1e-5 (they are in fact produced by the same operation
 trees, so most are bit-equal); gradients within 1e-5 of the gradient's scale
 (max |err| <= 1e-5 * max |ref| — the reference itself is run-to-run
 non-deterministic at this level because it accumulates with float atomics).
-Where oracle/_ref (the reference's own CUDA kernels, compiled in place) is
-present, it is used as a second, independent oracle.
+The reference's own CUDA kernels are a second, independent oracle: their outputs on
+the same inputs are stored in tests/golden/ref_cuda.npz (oracle/ref_golden.py).
 """
 import os
 
@@ -15,7 +15,7 @@ import pytest
 import torch
 
 import oracle
-from oracle import ref_cuda
+from oracle import ref_golden
 from kaolin_b200 import synthetic
 from kaolin_b200 import _C as b200_C
 from kaolin_b200.render.mesh import rasterize, dibr_soft_mask, dibr_rasterization
@@ -30,15 +30,6 @@ DEV = "cuda"
 # face); the reference's own kernels show the same deviation (printed below).
 GRAD_REL = 3e-5          # against the double-accumulating CPU oracle only
 GRAD_REL_REF = 1e-5      # against the reference's own CUDA kernels (north_star: "within 1e-5")
-
-
-def assert_grad_close(a, ref, tol=GRAD_REL_REF, what="grad"):
-    """max-normalised error <= tol AND element-wise allclose(rtol=tol, atol=tol * scale)."""
-    scale = max(float(np.abs(ref).max()), 1e-30)
-    e = float(np.abs(a - ref).max() / scale)
-    assert e <= tol, (what, e)
-    assert np.allclose(a, ref, rtol=tol, atol=tol * scale), what
-    return e
 
 
 def T(a, grad=False):
@@ -71,16 +62,20 @@ def _run_fused(fvz, fvi, fnz, ff, H, W, g_feat, g_soft, **kw):
     return N(feat), N(soft), N(idx), N(t_fvi.grad), N(t_ff.grad)
 
 
-@pytest.mark.parametrize("name", list(SCENES))
-def test_fused_dibr_vs_oracle(name):
+def fused_inputs(name):
     gen, H, W = SCENES[name]
     fvz, fvi, fnz = gen()
     B, F = fvz.shape[:2]
-    D = 3
-    ff = synthetic.random_features(B, F, D, seed=11)
+    ff = synthetic.random_features(B, F, 3, seed=11)
     rng = np.random.default_rng(12)
-    g_feat = rng.uniform(size=(B, H, W, D)).astype(np.float32)
+    g_feat = rng.uniform(size=(B, H, W, 3)).astype(np.float32)
     g_soft = rng.uniform(size=(B, H, W)).astype(np.float32)
+    return H, W, fvz, fvi, fnz, ff, g_feat, g_soft
+
+
+@pytest.mark.parametrize("name", list(SCENES))
+def test_fused_dibr_vs_oracle(name):
+    H, W, fvz, fvi, fnz, ff, g_feat, g_soft = fused_inputs(name)
     feat, soft, idx, g_fvi, g_ff = _run_fused(fvz, fvi, fnz, ff, H, W, g_feat, g_soft)
 
     o_feat, o_soft, o_idx, o_w = oracle.dibr_rasterization(H, W, fvz, fvi, ff, fnz, return_weights=True)
@@ -94,30 +89,23 @@ def test_fused_dibr_vs_oracle(name):
     assert rel_err(g_ff, o_gff) <= GRAD_REL, rel_err(g_ff, o_gff)
 
 
-@pytest.mark.skipif(not ref_cuda.available(), reason="oracle/_ref (reference CUDA build) not present")
 @pytest.mark.parametrize("name", list(SCENES))
 def test_fused_dibr_vs_reference_cuda(name):
-    """The reference's own kernels on the same GPU: face_idx bit-exact, 1e-5 elsewhere."""
-    gen, H, W = SCENES[name]
-    fvz, fvi, fnz = gen()
-    B, F = fvz.shape[:2]
-    ff = synthetic.random_features(B, F, 3, seed=11)
-    rng = np.random.default_rng(12)
-    g_feat = rng.uniform(size=(B, H, W, 3)).astype(np.float32)
-    g_soft = rng.uniform(size=(B, H, W)).astype(np.float32)
+    """The reference's own kernels on the same inputs: face_idx bit-exact, 1e-5 elsewhere."""
+    H, W, fvz, fvi, fnz, ff, g_feat, g_soft = fused_inputs(name)
     feat, soft, idx, g_fvi, g_ff = _run_fused(fvz, fvi, fnz, ff, H, W, g_feat, g_soft)
-    r = ref_cuda.dibr_forward_backward(H, W, T(fvz), T(fvi), T(ff), T(fnz), T(g_feat), T(g_soft))
+    case = "fused/" + name
     o_feat, o_soft, o_idx, o_w = oracle.dibr_rasterization(H, W, fvz, fvi, ff, fnz, return_weights=True)
     o_gxy, o_gff, _, _ = oracle.dibr_rasterization_backward(g_feat, g_soft, o_idx, o_w, fvi, ff)
+    o_rows, r_rows = ref_golden.sampled(case, "grad_fvi", o_gxy)
     print(f"\n[{name}] grad_fvi rel err vs double-accumulated oracle: ours {rel_err(g_fvi, o_gxy):.2e}, "
-          f"reference CUDA {rel_err(N(r['grad_fvi']), o_gxy):.2e}; ours vs reference CUDA "
-          f"{rel_err(g_fvi, N(r['grad_fvi'])):.2e}; soft_mask bit-equal to reference: "
-          f"{float((soft == N(r['soft_mask'])).mean()):.4f}")
-    assert np.array_equal(idx, N(r["face_idx"]))
-    np.testing.assert_allclose(feat, N(r["features"]), rtol=0, atol=1e-5)
-    np.testing.assert_allclose(soft, N(r["soft_mask"]), rtol=0, atol=1e-5)
-    assert_grad_close(g_fvi, N(r["grad_fvi"]), what="grad_fvi")     # both sides accumulate in fp32 atomics
-    assert_grad_close(g_ff, N(r["grad_ff"]), what="grad_ff")
+          f"reference CUDA {np.abs(r_rows - o_rows).max() / np.abs(o_gxy).max():.2e} (sampled); "
+          f"ours vs reference CUDA {ref_golden.rel_err(case, 'grad_fvi', g_fvi):.2e} (sampled)")
+    ref_golden.assert_equal(case, "face_idx", idx)
+    assert ref_golden.max_abs_err(case, "features", feat) <= 1e-5
+    assert ref_golden.max_abs_err(case, "soft_mask", soft) <= 1e-5
+    ref_golden.assert_grad_close(case, "grad_fvi", g_fvi, GRAD_REL_REF)     # both sides accumulate in fp32 atomics
+    ref_golden.assert_grad_close(case, "grad_ff", g_ff, GRAD_REL_REF)
 
 
 CONFIG_CASES = {
@@ -132,9 +120,7 @@ CONFIG_CASES = {
 }
 
 
-@pytest.mark.skipif(not ref_cuda.available(), reason="oracle/_ref (reference CUDA build) not present")
-@pytest.mark.parametrize("name", list(CONFIG_CASES))
-def test_baseline_configs_vs_reference_cuda(name):
+def config_inputs(name):
     B, level, H, W, jitter = CONFIG_CASES[name]
     fvz, fvi, fnz = synthetic.icosphere_views(B, level, seed=1234, jitter=jitter, same_mesh=(level >= 8))
     F = fvz.shape[1]
@@ -142,22 +128,26 @@ def test_baseline_configs_vs_reference_cuda(name):
     gen = torch.Generator(device=DEV); gen.manual_seed(7)
     g_feat = torch.rand((B, H, W, 3), device=DEV, generator=gen)
     g_soft = torch.rand((B, H, W), device=DEV, generator=gen)
-    t_fvz, t_fnz = T(fvz), T(fnz)
-    t_fvi, t_ff = T(fvi, True), T(ff, True)
+    return H, W, T(fvz), T(fvi), T(ff), T(fnz), g_feat, g_soft
+
+
+@pytest.mark.parametrize("name", list(CONFIG_CASES))
+def test_baseline_configs_vs_reference_cuda(name):
+    H, W, t_fvz, t_fvi, t_ff, t_fnz, g_feat, g_soft = config_inputs(name)
+    t_fvi.requires_grad_(True); t_ff.requires_grad_(True)
     feat, soft, idx = dibr_rasterization(H, W, t_fvz, t_fvi, t_ff, t_fnz)
     torch.autograd.backward([feat, soft], [g_feat, g_soft])
-    r = ref_cuda.dibr_forward_backward(H, W, t_fvz, t_fvi.detach(), t_ff.detach(), t_fnz, g_feat, g_soft)
-    assert torch.equal(idx, r["face_idx"])                                   # bit-exact
+    case = "config/" + name
+    ref_golden.assert_equal(case, "face_idx", idx)                           # bit-exact
     assert 0.2 < (idx >= 0).float().mean().item() < 0.9
-    assert (feat - r["features"]).abs().max().item() <= 1e-5
-    assert (soft - r["soft_mask"]).abs().max().item() <= 1e-5
-    bit_equal = (soft == r["soft_mask"]).float().mean().item()
-    e_xy = rel_err(N(t_fvi.grad), N(r["grad_fvi"]))
-    e_ff = rel_err(N(t_ff.grad), N(r["grad_ff"]))
-    print(f"\n[{name}] face_idx exact; soft_mask bit-equal {bit_equal:.6f}; grad rel err fvi {e_xy:.2e} ff {e_ff:.2e}")
+    assert ref_golden.max_abs_err(case, "features", feat) <= 1e-5
+    assert ref_golden.max_abs_err(case, "soft_mask", soft) <= 1e-5
+    mine, ref = ref_golden.sampled(case, "soft_mask", soft)
+    bit_equal = float((mine == ref).mean())
+    e_xy = ref_golden.assert_grad_close(case, "grad_fvi", t_fvi.grad, GRAD_REL_REF)
+    e_ff = ref_golden.assert_grad_close(case, "grad_ff", t_ff.grad, GRAD_REL_REF)
+    print(f"\n[{name}] face_idx exact; soft_mask bit-equal {bit_equal:.6f} (sampled); grad rel err fvi {e_xy:.2e} ff {e_ff:.2e}")
     assert bit_equal > 0.9999
-    assert_grad_close(N(t_fvi.grad), N(r["grad_fvi"]), what="grad_fvi")
-    assert_grad_close(N(t_ff.grad), N(r["grad_ff"]), what="grad_ff")
 
 
 def test_two_call_backward_with_feature_grad_hook_equals_fused():
@@ -211,13 +201,7 @@ def test_backward_through_one_output_only():
     assert np.abs(out["soft"][0]).max() > 0 and np.abs(out["feat"][0]).max() > 0
 
 
-@pytest.mark.skipif(not ref_cuda.available(), reason="oracle/_ref (reference CUDA build) not present")
-@pytest.mark.parametrize("D", [3, 5])
-def test_bf16_feature_storage_vs_reference_cuda(D):
-    """BASELINE configs[3]: bf16 face_features / features / grad_features, fp32 arithmetic.
-    The interpolated features equal the reference's fp32 result (on the same bf16-rounded
-    inputs) rounded once to bf16; everything geometric is unchanged."""
-    from kaolin_b200.render.mesh import _host
+def bf16_inputs(D):
     fvz, fvi, fnz = synthetic.icosphere_views(2, 4, seed=21)
     B, F = fvz.shape[:2]
     H, W = 192, 176
@@ -225,27 +209,36 @@ def test_bf16_feature_storage_vs_reference_cuda(D):
     gen = torch.Generator(device=DEV); gen.manual_seed(9)
     g_feat16 = torch.rand((B, H, W, D), device=DEV, generator=gen).to(torch.bfloat16)
     g_soft = torch.rand((B, H, W), device=DEV, generator=gen)
-    t_fvz, t_fnz = T(fvz), T(fnz)
-    t_fvi, t_ff = T(fvi, True), ff16.clone().requires_grad_(True)
+    return H, W, T(fvz), T(fvi), ff16, T(fnz), g_feat16, g_soft
+
+
+@pytest.mark.parametrize("D", [3, 5])
+def test_bf16_feature_storage_vs_reference_cuda(D):
+    """BASELINE configs[3]: bf16 face_features / features / grad_features, fp32 arithmetic.
+    The interpolated features equal the reference's fp32 result (on the same bf16-rounded
+    inputs) rounded once to bf16; everything geometric is unchanged."""
+    from kaolin_b200.render.mesh import _host
+    H, W, t_fvz, t_fvi, ff16, t_fnz, g_feat16, g_soft = bf16_inputs(D)
+    t_fvi.requires_grad_(True)
+    t_ff = ff16.clone().requires_grad_(True)
     feat, soft, idx = dibr_rasterization(H, W, t_fvz, t_fvi, t_ff, t_fnz)
     assert feat.dtype == torch.bfloat16 and soft.dtype == torch.float32
     torch.autograd.backward([feat, soft], [g_feat16, g_soft])
     assert t_ff.grad.dtype == torch.bfloat16 and t_fvi.grad.dtype == torch.float32
-    r = ref_cuda.dibr_forward_backward(H, W, t_fvz, t_fvi.detach(), ff16.float(), t_fnz,
-                                       g_feat16.float(), g_soft)
-    assert torch.equal(idx, r["face_idx"])
-    assert torch.equal(soft, r["soft_mask"])
-    assert torch.equal(feat, r["features"].to(torch.bfloat16))            # one rounding, on store
-    assert rel_err(N(t_fvi.grad), N(r["grad_fvi"])) <= GRAD_REL_REF
-    assert rel_err(N(t_ff.grad.float()), N(r["grad_ff"])) <= 2.0 ** -8      # bf16 rounding of the result
+    case = f"bf16/D{D}"
+    ref_golden.assert_equal(case, "face_idx", idx)
+    ref_golden.assert_equal(case, "soft_mask", soft)
+    ref_golden.assert_equal(case, "features_bf16", feat)                  # one rounding, on store
+    assert ref_golden.rel_err(case, "grad_fvi", t_fvi.grad) <= GRAD_REL_REF
+    assert ref_golden.rel_err(case, "grad_ff", t_ff.grad) <= 2.0 ** -8      # bf16 rounding of the result
     # the C ABI returns the fp32 accumulation itself
     feat2, idx2, wts2, soft2, ws = _host.forward(3, H, W, t_fvz, t_fvi.detach(), ff16, t_fnz, None, 1000., 1e-8,
                                                  7000., 0.02 * 1000., 30)
     g_fvi, g_ff = _host.backward(H, W, g_feat16, g_soft, idx2, wts2, soft2, t_fvi.detach(), ff16, 1000., 1e-8,
                                  7000., 0.02 * 1000., 30, ws, True)
     assert g_ff.dtype == torch.float32 and torch.equal(feat2, feat)
-    assert rel_err(N(g_ff), N(r["grad_ff"])) <= GRAD_REL_REF
-    assert rel_err(N(g_fvi), N(r["grad_fvi"])) <= GRAD_REL_REF
+    assert ref_golden.rel_err(case, "grad_ff", g_ff) <= GRAD_REL_REF
+    assert ref_golden.rel_err(case, "grad_fvi", g_fvi) <= GRAD_REL_REF
     # rasterize alone, tuple features
     (a, b), idx3 = rasterize(H, W, t_fvz, t_fvi.detach(), [ff16[..., :2], ff16[..., 2:]], t_fnz >= 0.)
     assert torch.equal(idx3, idx) and torch.equal(torch.cat([a, b], -1), feat)
