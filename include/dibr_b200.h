@@ -10,6 +10,13 @@
  * Every output is fully written (no pre-zeroing needed).  Calls are asynchronous
  * on `stream` and never synchronise; they are re-entrant (no global state).
  *
+ * Alignment: every device tensor pointer (inputs and outputs) must be a multiple of
+ * DIBR_B200_ALIGNMENT (16) bytes; NULL is allowed where documented.  The kernels access caller
+ * tensors with 16-byte vector loads / stores and 16- or 8-byte cp.async copies, so a tensor
+ * view at a storage offset (e.g. buf[1:] of a float buffer, 4 bytes in) is rejected with
+ * DIBR_B200_EINVAL before anything is launched; copy it first.  The workspace is exempt (it
+ * is aligned internally) and so are host pointers (camera_proj_host, peer-push arrays).
+ *
  * Return value: 0 on success; DIBR_B200_E* (<0) for argument errors detected on
  * the host; a positive cudaError_t if a launch failed (cudaGetLastError()).
  *
@@ -29,11 +36,12 @@ extern "C" {
 #endif
 
 #define DIBR_B200_OK 0
-#define DIBR_B200_EINVAL (-1)      /* null pointer / non-positive size / bad flag */
+#define DIBR_B200_EINVAL (-1)      /* null or misaligned pointer / non-positive size / bad flag */
 #define DIBR_B200_EWORKSPACE (-3)  /* workspace_bytes too small */
 #define DIBR_B200_ESIZE (-4)       /* image larger than 16384 px or index overflow */
 
 #define DIBR_B200_MAX_IMAGE_DIM 16384
+#define DIBR_B200_ALIGNMENT 16     /* bytes, every device tensor pointer (see above) */
 
 /* forward `mode` bits */
 #define DIBR_B200_RASTER 1     /* compute face_idx / weights / features */

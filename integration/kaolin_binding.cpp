@@ -35,6 +35,12 @@ dibr_b200_stream_t current_stream() {
   return reinterpret_cast<dibr_b200_stream_t>(at::cuda::getCurrentCUDAStream().stream());
 }
 
+// include/dibr_b200.h: every tensor pointer 16-byte aligned.  A contiguous view at a storage
+// offset passes the reference's checks, so such an input is copied first.
+at::Tensor aligned(const at::Tensor& t) {
+  return reinterpret_cast<uintptr_t>(t.data_ptr()) % DIBR_B200_ALIGNMENT ? t.clone(at::MemoryFormat::Contiguous) : t;
+}
+
 at::Tensor workspace(const at::Tensor& like, int batch, int64_t faces, int height, int width) {
   const size_t n = dibr_b200_workspace_bytes(batch, faces, height, width);
   TORCH_CHECK(n > 0, "libdibr_b200: unsupported problem size");
@@ -65,14 +71,16 @@ std::vector<at::Tensor> packed_rasterize_forward_cuda(
   at::checkSize(__func__, first_arg, {batch + 1});
   check_float(__func__, face_vertices_z);
   const at::cuda::OptionalCUDAGuard guard(at::device_of(face_vertices_z));
+  const at::Tensor z = aligned(face_vertices_z), xy = aligned(face_vertices_image), bb = aligned(face_bboxes),
+                   ff = aligned(face_features), first = aligned(first_idx_face_per_mesh);
   auto opt = face_vertices_z.options();
   at::Tensor idx = at::empty({batch, height, width}, opt.dtype(at::kLong));
   at::Tensor w = at::empty({batch, height, width, 3}, opt);
   at::Tensor out = at::empty({batch, height, width, D}, opt);
   at::Tensor ws = workspace(face_vertices_z, batch, num_faces, height, width);
   check_status(__func__, dibr_b200_packed_rasterize_forward(
-      batch, num_faces, height, width, D, face_vertices_z.data_ptr<float>(), face_vertices_image.data_ptr<float>(),
-      face_bboxes.data_ptr<float>(), face_features.data_ptr<float>(), first_idx_face_per_mesh.data_ptr<int64_t>(),
+      batch, num_faces, height, width, D, z.data_ptr<float>(), xy.data_ptr<float>(),
+      bb.data_ptr<float>(), ff.data_ptr<float>(), first.data_ptr<int64_t>(),
       multiplier, eps, out.data_ptr<float>(), idx.data_ptr<int64_t>(), w.data_ptr<float>(), ws.data_ptr(),
       static_cast<size_t>(ws.numel()), current_stream()));
   return {out, idx, w};
@@ -101,14 +109,16 @@ std::vector<at::Tensor> rasterize_backward_cuda(
   at::checkSize(__func__, ff_arg, {batch, F, 3, D});
   check_float(__func__, grad_interpolated_features);
   const at::cuda::OptionalCUDAGuard guard(at::device_of(grad_interpolated_features));
+  const at::Tensor g = aligned(grad_interpolated_features), idx = aligned(selected_face_idx),
+                   w = aligned(output_weights), xy = aligned(face_vertices_image), ff = aligned(face_features);
   at::Tensor g_xy = at::empty_like(face_vertices_image);
   at::Tensor g_ff = at::empty_like(face_features);
   // the fused entry point with a workspace takes the row-walk scatter kernel
   at::Tensor ws = workspace(face_vertices_image, batch, static_cast<int64_t>(batch) * F, height, width);
   check_status(__func__, dibr_b200_backward(
-      batch, F, height, width, D, grad_interpolated_features.data_ptr<float>(), nullptr,
-      selected_face_idx.data_ptr<int64_t>(), output_weights.data_ptr<float>(), nullptr,
-      face_vertices_image.data_ptr<float>(), face_features.data_ptr<float>(), 1.f, eps, 0.f, 0.f, 0,
+      batch, F, height, width, D, g.data_ptr<float>(), nullptr,
+      idx.data_ptr<int64_t>(), w.data_ptr<float>(), nullptr,
+      xy.data_ptr<float>(), ff.data_ptr<float>(), 1.f, eps, 0.f, 0.f, 0,
       g_xy.data_ptr<float>(), g_ff.data_ptr<float>(), ws.data_ptr(), static_cast<size_t>(ws.numel()), 0,
       current_stream()));
   return {g_xy, g_ff};
@@ -131,6 +141,7 @@ std::vector<at::Tensor> dibr_soft_mask_forward_cuda(
   at::checkSize(__func__, idx_arg, {batch, height, width});
   check_float(__func__, face_vertices_image);
   const at::cuda::OptionalCUDAGuard guard(at::device_of(face_vertices_image));
+  const at::Tensor xy = aligned(face_vertices_image), bb = aligned(face_large_bboxes), idx = aligned(selected_face_idx);
   auto opt = face_vertices_image.options();
   at::Tensor soft = at::empty({batch, height, width}, opt);
   at::Tensor prob = at::empty({batch, height, width, knum}, opt);
@@ -138,8 +149,8 @@ std::vector<at::Tensor> dibr_soft_mask_forward_cuda(
   at::Tensor ctype = at::empty({batch, height, width, knum}, opt.dtype(at::kByte));
   at::Tensor ws = workspace(face_vertices_image, batch, static_cast<int64_t>(batch) * F, height, width);
   check_status(__func__, dibr_b200_soft_mask_forward(
-      batch, F, height, width, knum, face_vertices_image.data_ptr<float>(), face_large_bboxes.data_ptr<float>(),
-      selected_face_idx.data_ptr<int64_t>(), sigmainv, multiplier, soft.data_ptr<float>(), prob.data_ptr<float>(),
+      batch, F, height, width, knum, xy.data_ptr<float>(), bb.data_ptr<float>(),
+      idx.data_ptr<int64_t>(), sigmainv, multiplier, soft.data_ptr<float>(), prob.data_ptr<float>(),
       cidx.data_ptr<int64_t>(), ctype.data_ptr<uint8_t>(), ws.data_ptr(), static_cast<size_t>(ws.numel()),
       current_stream()));
   return {soft, prob, cidx, ctype};
@@ -170,11 +181,14 @@ at::Tensor dibr_soft_mask_backward_cuda(
   at::checkSize(__func__, xy_arg, {batch, F, 3, 2});
   check_float(__func__, grad_soft_mask);
   const at::cuda::OptionalCUDAGuard guard(at::device_of(grad_soft_mask));
+  const at::Tensor g = aligned(grad_soft_mask), soft = aligned(soft_mask), idx = aligned(selected_face_idx),
+                   prob = aligned(close_face_prob), cidx = aligned(close_face_idx),
+                   ctype = aligned(close_face_dist_type), xy = aligned(face_vertices_image);
   at::Tensor g_xy = at::empty_like(face_vertices_image);
   check_status(__func__, dibr_b200_soft_mask_backward(
-      batch, F, height, width, knum, grad_soft_mask.data_ptr<float>(), soft_mask.data_ptr<float>(),
-      selected_face_idx.data_ptr<int64_t>(), close_face_prob.data_ptr<float>(), close_face_idx.data_ptr<int64_t>(),
-      close_face_dist_type.data_ptr<uint8_t>(), face_vertices_image.data_ptr<float>(), sigmainv, multiplier,
+      batch, F, height, width, knum, g.data_ptr<float>(), soft.data_ptr<float>(),
+      idx.data_ptr<int64_t>(), prob.data_ptr<float>(), cidx.data_ptr<int64_t>(),
+      ctype.data_ptr<uint8_t>(), xy.data_ptr<float>(), sigmainv, multiplier,
       g_xy.data_ptr<float>(), current_stream()));
   return g_xy;
 }

@@ -19,6 +19,13 @@ def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
+def _aligned(*ts):
+    """The tensors, each copied when its data pointer is not 16-byte aligned (include/dibr_b200.h:
+    the C ABI rejects it; the reference's wrappers take contiguous views at any storage offset)."""
+    from .render.mesh._host import aligned
+    return [aligned(t) for t in ts]
+
+
 def _stream(dev):
     return ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
@@ -94,6 +101,8 @@ def packed_rasterize_forward_cuda(height, width, face_vertices_z, face_vertices_
     _check_size(fn, "first_idx_face_per_mesh", first_idx_face_per_mesh, (batch_size + 1,))
     if first_idx_face_per_mesh.dtype != torch.int64:
         raise RuntimeError(f"{fn}: first_idx_face_per_mesh must be a LongTensor")
+    face_vertices_z, face_vertices_image, face_bboxes, face_features, first_idx_face_per_mesh = _aligned(
+        face_vertices_z, face_vertices_image, face_bboxes, face_features, first_idx_face_per_mesh)
     idx = torch.empty((batch_size, height, width), dtype=torch.int64, device=dev)
     w = torch.empty((batch_size, height, width, 3), dtype=torch.float32, device=dev)
     out = torch.empty((batch_size, height, width, feat_dim), dtype=torch.float32, device=dev)
@@ -126,6 +135,8 @@ def rasterize_backward_cuda(grad_interpolated_features, interpolated_features, s
     _check_size(fn, "output_weights", output_weights, (B, H, W, 3))
     _check_size(fn, "face_vertices_image", face_vertices_image, (B, F, 3, 2))
     _check_size(fn, "face_features", face_features, (B, F, 3, D))
+    grad_interpolated_features, selected_face_idx, output_weights, face_vertices_image, face_features = _aligned(
+        grad_interpolated_features, selected_face_idx, output_weights, face_vertices_image, face_features)
     g_xy = torch.empty_like(face_vertices_image)
     g_ff = torch.empty_like(face_features)
     with torch.cuda.device(dev):
@@ -150,6 +161,8 @@ def dibr_soft_mask_forward_cuda(face_vertices_image, face_large_bboxes, selected
     _check_size(fn, "face_vertices_image", face_vertices_image, (B, F, 3, 2))
     _check_size(fn, "face_bboxes", face_large_bboxes, (B, F, 4))
     _check_size(fn, "selected_face_idx", selected_face_idx, (B, H, W))
+    face_vertices_image, face_large_bboxes, selected_face_idx = _aligned(
+        face_vertices_image, face_large_bboxes, selected_face_idx)
     soft = torch.empty((B, H, W), dtype=torch.float32, device=dev)
     prob = torch.empty((B, H, W, knum), dtype=torch.float32, device=dev)
     cidx = torch.empty((B, H, W, knum), dtype=torch.int64, device=dev)
@@ -185,8 +198,10 @@ def dibr_soft_mask_backward_cuda(grad_soft_mask, soft_mask, selected_face_idx, c
     _check_size(fn, "close_face_idx", close_face_idx, (B, H, W, K))
     _check_size(fn, "close_face_dist_type", close_face_dist_type, (B, H, W, K))
     _check_size(fn, "face_vertices_image", face_vertices_image, (B, F, 3, 2))
+    grad_soft_mask, soft_mask, close_face_prob, close_face_idx, close_face_dist_type, face_vertices_image = _aligned(
+        grad_soft_mask, soft_mask, close_face_prob, close_face_idx, close_face_dist_type, face_vertices_image)
     g = torch.empty_like(face_vertices_image)
-    sel = selected_face_idx.contiguous()
+    sel, = _aligned(selected_face_idx.contiguous())
     with torch.cuda.device(dev):
         st = _lib.lib().dibr_b200_soft_mask_backward(
             B, F, H, W, K, _ptr(grad_soft_mask), _ptr(soft_mask), _ptr(sel), _ptr(close_face_prob),
@@ -211,6 +226,8 @@ def deftet_sparse_render_forward_cuda(face_vertices_z, face_vertices_image, face
     _check_size(fn, "face_bboxes", face_bboxes, (B, F, 4))
     _check_size(fn, "pixel_coords", pixel_coords, (B, P, 2))
     _check_size(fn, "pixel_depth_ranges", pixel_depth_ranges, (B, P, 2))
+    face_vertices_z, face_vertices_image, face_bboxes, pixel_coords, pixel_depth_ranges = _aligned(
+        face_vertices_z, face_vertices_image, face_bboxes, pixel_coords, pixel_depth_ranges)
     idx = torch.empty((B, P, knum), dtype=torch.int64, device=dev)
     depth = torch.empty((B, P, knum), dtype=torch.float32, device=dev)
     w0 = torch.empty((B, P, knum), dtype=torch.float32, device=dev)
@@ -240,6 +257,8 @@ def deftet_sparse_render_backward_cuda(grad_interpolated_features, face_idx, wei
     _check_size(fn, "weights", weights, (B, P, K, 3))
     _check_size(fn, "face_vertices_image", face_vertices_image, (B, F, 3, 2))
     _check_size(fn, "face_features", face_features, (B, F, 3, D))
+    grad_interpolated_features, face_idx, weights, face_vertices_image, face_features = _aligned(
+        grad_interpolated_features, face_idx, weights, face_vertices_image, face_features)
     g_xy = torch.empty_like(face_vertices_image)
     g_ff = torch.empty_like(face_features)
     with torch.cuda.device(dev):

@@ -22,6 +22,7 @@ NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a",
               "-Xcompiler", "-fPIC", "-shared"]
 
 EINVAL, EWORKSPACE, ESIZE = -1, -3, -4
+ALIGNMENT = 16                      # DIBR_B200_ALIGNMENT: bytes, every device tensor pointer
 RASTER, SOFT_MASK = 1, 2
 BINS_VALID, ACCUMULATE = 1, 2      # dibr_b200_backward flags
 
@@ -144,7 +145,7 @@ def check(status, what):
     if status == 0:
         return
     if status == EINVAL:
-        raise RuntimeError(f"{what}: invalid argument (null pointer, non-positive size or multiplier)")
+        raise RuntimeError(f"{what}: invalid argument (null or misaligned pointer, non-positive size or multiplier)")
     if status == EWORKSPACE:
         raise RuntimeError(f"{what}: workspace too small")
     if status == ESIZE:

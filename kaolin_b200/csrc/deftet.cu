@@ -30,6 +30,11 @@ namespace {
 
 using namespace dibr;
 
+// Any tensor pointer not DIBR_B200_ALIGNMENT-byte aligned (NULL is aligned): bboxes are read as
+// float4, coordinates as float2.
+template <typename... P>
+bool misaligned(P... p) { return ((((uintptr_t)p) | ... | (uintptr_t)0) & (DIBR_B200_ALIGNMENT - 1)) != 0; }
+
 constexpr int kMaxCells = 16;     // cells a face may be inserted in; wider faces -> the view's wide list
 constexpr int kHitCap = 128;      // hits a point can collect before it takes the ordered scan
 constexpr int kWarps = 8;         // points per CTA
@@ -332,6 +337,9 @@ int dibr_b200_deftet_sparse_render_forward(int batch, int num_faces, int num_pix
   if (batch <= 0 || num_faces < 0 || num_pixels < 0 || knum <= 0) return DIBR_B200_EINVAL;
   if (!pixel_coords || !render_ranges || !face_idx || !pixel_depth || !w0 || !w1 || !workspace) return DIBR_B200_EINVAL;
   if (num_faces > 0 && (!face_vertices_z || !face_vertices_image || !face_bboxes)) return DIBR_B200_EINVAL;
+  if (misaligned(face_vertices_z, face_vertices_image, face_bboxes, pixel_coords, render_ranges, face_idx,
+                 pixel_depth, w0, w1))
+    return DIBR_B200_EINVAL;
   if ((int64_t)batch * num_pixels * knum >= (int64_t)1 << 40 || (int64_t)num_faces * kMaxCells >= 0x7fffffffLL) return DIBR_B200_ESIZE;
   const Layout L = layout_for(batch, num_faces);
   char* p = (char*)align_up((size_t)workspace, 256);
@@ -373,6 +381,9 @@ int dibr_b200_deftet_sparse_render_backward(int batch, int num_faces, int num_pi
                                             dibr_b200_stream_t stream) {
   if (batch <= 0 || num_faces < 0 || num_pixels < 0 || knum <= 0 || feat_dim < 0) return DIBR_B200_EINVAL;
   if (!grad_face_vertices_image || (feat_dim > 0 && !grad_face_features)) return DIBR_B200_EINVAL;
+  if (misaligned(grad_interpolated_features, face_idx, weights, face_vertices_image, face_features,
+                 grad_face_vertices_image, grad_face_features))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t nf = (int64_t)batch * num_faces;
   cudaError_t e = cudaMemsetAsync(grad_face_vertices_image, 0, (size_t)nf * 6 * sizeof(float), st);

@@ -40,6 +40,11 @@ namespace {
 
 using namespace dibr;
 
+// Any tensor pointer not DIBR_B200_ALIGNMENT-byte aligned (NULL is aligned): the kernels read and
+// write caller tensors with 16-byte vector and cp.async accesses.
+template <typename... P>
+bool misaligned(P... p) { return ((((uintptr_t)p) | ... | (uintptr_t)0) & (DIBR_B200_ALIGNMENT - 1)) != 0; }
+
 constexpr int kTile = 16;
 constexpr int kThreads = 256;
 constexpr int kChunk = 256;
@@ -2786,6 +2791,9 @@ int dibr_b200_forward_f64(int batch, int num_faces, int height, int width, int f
                  (num_faces > 0 && !face_vertices_z)))
     return DIBR_B200_EINVAL;
   if (soft && (!soft_mask || knum <= 0)) return DIBR_B200_EINVAL;
+  if (misaligned(face_vertices_z, face_vertices_image, face_features, face_normals_z, valid_faces,
+                 interpolated_features, face_idx, output_weights, soft_mask))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   F64Args a;
   rc = f64_setup(a, batch, num_faces, height, width, face_vertices_image, face_normals_z, valid_faces, multiplier,
@@ -2814,6 +2822,9 @@ int dibr_b200_backward_f64(int batch, int num_faces, int height, int width, int 
   const bool run_raster = grad_features && feat_dim > 0;
   if (run_raster && NF > 0 && (!output_weights || !face_features || !grad_face_features)) return DIBR_B200_EINVAL;
   if (grad_soft_mask && (!soft_mask || knum <= 0)) return DIBR_B200_EINVAL;
+  if (misaligned(grad_features, grad_soft_mask, face_idx, output_weights, soft_mask, face_vertices_image,
+                 face_features, grad_face_vertices_image, grad_face_features))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   cudaError_t e = cudaMemsetAsync(grad_face_vertices_image, 0, (size_t)NF * 6 * sizeof(double), st);
   if (e != cudaSuccess) return (int)e;
@@ -2900,6 +2911,9 @@ static int forward_impl(int batch, int num_faces, int height, int width, int fea
                  (num_faces > 0 && !face_vertices_z)))
     return DIBR_B200_EINVAL;
   if (soft && (!soft_mask || knum <= 0)) return DIBR_B200_EINVAL;
+  if (misaligned(face_vertices_z, face_vertices_image, face_features, face_normals_z, valid_faces,
+                 interpolated_features, face_idx, output_weights, soft_mask))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   FwdArgs a;
   Scene& s = a.s;
@@ -2963,6 +2977,9 @@ static int backward_impl(int batch, int num_faces, int height, int width, int fe
   if (!face_idx || !grad_face_vertices_image || num_faces < 0 || feat_dim < 0) return DIBR_B200_EINVAL;
   if (num_faces > 0 && !face_vertices_image) return DIBR_B200_EINVAL;
   if (view_begin < 0 || view_end > batch || view_begin >= view_end) return DIBR_B200_EINVAL;
+  if (misaligned(grad_features, grad_soft_mask, face_idx, output_weights, soft_mask, face_vertices_image,
+                 face_features, grad_face_vertices_image, grad_face_features))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   cudaError_t e = cudaSuccess;
   const bool run_raster = grad_features && feat_dim > 0;
@@ -3099,6 +3116,9 @@ int dibr_b200_packed_rasterize_forward(int batch, int64_t total_faces, int heigh
   if (!selected_face_idx || !output_weights || !first_idx_face_per_mesh || feat_dim < 0) return DIBR_B200_EINVAL;
   if (feat_dim > 0 && (!interpolated_features || (total_faces > 0 && !face_features))) return DIBR_B200_EINVAL;
   if (total_faces > 0 && (!face_vertices_z || !face_vertices_image || !face_bboxes)) return DIBR_B200_EINVAL;
+  if (misaligned(face_vertices_z, face_vertices_image, face_bboxes, face_features, first_idx_face_per_mesh,
+                 interpolated_features, selected_face_idx, output_weights))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   FwdArgs a;
   Scene& s = a.s;
@@ -3145,6 +3165,9 @@ int dibr_b200_soft_mask_forward(int batch, int num_faces, int height, int width,
   const bool lists = close_face_prob || close_face_idx || close_face_dist_type;
   if (lists && !(close_face_prob && close_face_idx && close_face_dist_type)) return DIBR_B200_EINVAL;
   if (lists && (int64_t)batch * height * width * knum < 0) return DIBR_B200_ESIZE;
+  if (misaligned(face_vertices_image, face_large_bboxes, selected_face_idx, soft_mask, close_face_prob,
+                 close_face_idx, close_face_dist_type))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   FwdArgs a;
   Scene& s = a.s;
@@ -3177,6 +3200,9 @@ int dibr_b200_soft_mask_backward(int batch, int num_faces, int height, int width
       !close_face_dist_type || !grad_face_vertices_image || knum <= 0 || !(multiplier > 0.f))
     return DIBR_B200_EINVAL;
   if (num_faces > 0 && !face_vertices_image) return DIBR_B200_EINVAL;
+  if (misaligned(grad_soft_mask, soft_mask, selected_face_idx, close_face_prob, close_face_idx,
+                 close_face_dist_type, face_vertices_image, grad_face_vertices_image))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   cudaError_t e = cudaMemsetAsync(grad_face_vertices_image, 0, (size_t)NF * 6 * sizeof(float), st);
   if (e != cudaSuccess) return (int)e;

@@ -25,6 +25,11 @@
 
 namespace {
 
+// Any tensor pointer not DIBR_B200_ALIGNMENT-byte aligned (NULL is aligned).  Texture coordinates
+// and their gradient are read and written as float2; the rule is the same for every entry point.
+template <typename... P>
+bool misaligned(P... p) { return ((((uintptr_t)p) | ... | (uintptr_t)0) & (DIBR_B200_ALIGNMENT - 1)) != 0; }
+
 // ---------------------------------------------------------------------------
 // prepare_vertices
 struct Cam {
@@ -335,6 +340,9 @@ int dibr_b200_prepare_vertices_forward(int batch, int num_vertices, int num_face
                                        dibr_b200_stream_t stream) {
   if (batch <= 0 || num_vertices <= 0 || num_faces < 0) return DIBR_B200_EINVAL;
   if (!vertices || !faces || !face_vertices_camera || !face_vertices_image || !face_normals) return DIBR_B200_EINVAL;
+  if (misaligned(vertices, faces, camera_transform, camera_rot, camera_trans, face_vertices_camera,
+                 face_vertices_image, face_normals))
+    return DIBR_B200_EINVAL;
   Cam c;
   const int rc = make_cam(c, camera_transform, camera_rot, camera_trans, camera_proj_host);
   if (rc) return rc;
@@ -353,6 +361,9 @@ int dibr_b200_prepare_vertices_backward(int batch, int num_vertices, int num_fac
                                         float* grad_vertices_camera, dibr_b200_stream_t stream) {
   if (batch <= 0 || num_vertices <= 0 || num_faces < 0) return DIBR_B200_EINVAL;
   if (!vertices || !faces || !grad_vertices_camera) return DIBR_B200_EINVAL;
+  if (misaligned(vertices, faces, camera_transform, camera_rot, camera_trans, grad_face_vertices_camera,
+                 grad_face_vertices_image, grad_face_normals, grad_vertices_camera))
+    return DIBR_B200_EINVAL;
   Cam c;
   const int rc = make_cam(c, camera_transform, camera_rot, camera_trans, camera_proj_host);
   if (rc) return rc;
@@ -372,6 +383,7 @@ int dibr_b200_texture_mapping_forward(int batch, int64_t num_points, int channel
                                       float* out, dibr_b200_stream_t stream) {
   if (batch <= 0 || num_points < 0 || channels <= 0 || tex_height <= 0 || tex_width <= 0) return DIBR_B200_EINVAL;
   if (!texture_coordinates || !texture_maps || !out) return DIBR_B200_EINVAL;
+  if (misaligned(texture_coordinates, texture_maps, out)) return DIBR_B200_EINVAL;
   const int64_t n = (int64_t)batch * num_points;
   if (n == 0) return 0;
   const unsigned blocks = (unsigned)((n + 255) / 256);
@@ -386,6 +398,8 @@ int dibr_b200_texture_mapping_backward(int batch, int64_t num_points, int channe
                                        float* grad_texture_coordinates, dibr_b200_stream_t stream) {
   if (batch <= 0 || num_points < 0 || channels <= 0 || tex_height <= 0 || tex_width <= 0) return DIBR_B200_EINVAL;
   if (!texture_coordinates || !texture_maps || !grad_out) return DIBR_B200_EINVAL;
+  if (misaligned(texture_coordinates, texture_maps, grad_out, grad_texture_maps, grad_texture_coordinates))
+    return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   if (grad_texture_maps) {
     cudaError_t e = cudaMemsetAsync(grad_texture_maps, 0, (size_t)batch * channels * tex_height * tex_width * sizeof(float), st);
@@ -402,6 +416,7 @@ int dibr_b200_texture_mapping_backward(int batch, int64_t num_points, int channe
 int dibr_b200_mask_iou_forward(int batch, int64_t pixels_per_view, const float* lhs_mask, const float* rhs_mask,
                                float* sums, float* loss, dibr_b200_stream_t stream) {
   if (batch <= 0 || batch > 65535 || pixels_per_view <= 0 || !lhs_mask || !rhs_mask || !sums || !loss) return DIBR_B200_EINVAL;
+  if (misaligned(lhs_mask, rhs_mask, sums, loss)) return DIBR_B200_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   cudaError_t e = cudaMemsetAsync(sums, 0, (size_t)batch * 2 * sizeof(float), st);
   if (e != cudaSuccess) return (int)e;
@@ -416,6 +431,7 @@ int dibr_b200_mask_iou_backward(int batch, int64_t pixels_per_view, const float*
                                 const float* sums, const float* grad_loss, float* grad_lhs, float* grad_rhs,
                                 dibr_b200_stream_t stream) {
   if (batch <= 0 || batch > 65535 || pixels_per_view <= 0 || !lhs_mask || !rhs_mask || !sums || !grad_loss) return DIBR_B200_EINVAL;
+  if (misaligned(lhs_mask, rhs_mask, sums, grad_loss, grad_lhs, grad_rhs)) return DIBR_B200_EINVAL;
   int64_t bx = (pixels_per_view + 256 * 8 - 1) / (256 * 8);
   if (bx > 1184) bx = 1184;
   mask_iou_bwd_kernel<<<dim3((unsigned)bx, (unsigned)batch), 256, 0, (cudaStream_t)stream>>>(

@@ -14,7 +14,7 @@ __all__ = ["mask_iou"]
 class MaskIouB200(Function):
     @staticmethod
     def forward(ctx, lhs_mask, rhs_mask):
-        l, r = lhs_mask.contiguous(), rhs_mask.contiguous()
+        l, r = _host.aligned(lhs_mask.contiguous()), _host.aligned(rhs_mask.contiguous())
         B = l.shape[0]
         hw = l.numel() // B
         sums = torch.empty((B, 2), dtype=torch.float32, device=l.device)
@@ -33,7 +33,7 @@ class MaskIouB200(Function):
         hw = l.numel() // B
         g_l = torch.empty_like(l) if ctx.needs_input_grad[0] else None
         g_r = torch.empty_like(r) if ctx.needs_input_grad[1] else None
-        g = g_loss.contiguous().to(torch.float32)
+        g = _host.aligned(g_loss.contiguous().to(torch.float32))
         with torch.cuda.device(l.device):
             st = _lib.lib().dibr_b200_mask_iou_backward(B, hw, _host.ptr(l), _host.ptr(r), _host.ptr(sums),
                                                         _host.ptr(g), _host.ptr(g_l), _host.ptr(g_r),

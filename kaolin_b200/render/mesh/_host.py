@@ -12,6 +12,17 @@ def ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
+def aligned(t):
+    """``t`` itself, or a copy when its data pointer is not a multiple of _lib.ALIGNMENT bytes.
+
+    The C ABI rejects such pointers (the kernels use 16-byte vector and cp.async accesses); a
+    contiguous view at a storage offset, such as an upstream gradient ``buf[1:].view(...)`` that
+    autograd passes through unchanged, gets there otherwise."""
+    if t is None or t.data_ptr() % _lib.ALIGNMENT == 0:
+        return t
+    return t.clone(memory_format=torch.contiguous_format)
+
+
 def stream_ptr(device):
     return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
@@ -93,6 +104,7 @@ def workspace(batch, total_faces, height, width, device, knum=0):
 def forward(mode, height, width, fvz, fvi, ff, fnz, valid_u8, multiplier, eps,
             sigmainv, boxlen_m, knum, face_idx_in=None):
     """Calls dibr_b200_forward; returns (feat, face_idx, weights, soft, workspace)."""
+    fvz, fvi, ff, fnz, valid_u8, face_idx_in = map(aligned, (fvz, fvi, ff, fnz, valid_u8, face_idx_in))
     dev = fvi.device
     B, F = fvi.shape[0], fvi.shape[1]
     D = 0 if ff is None else ff.shape[-1]
@@ -148,12 +160,14 @@ def backward(height, width, g_feat, g_soft, face_idx, wts, soft, fvi, ff, multip
     ``views=(v0, v1)`` restricts the call to those views of the batch (dibr_b200_backward_views: all
     tensors stay the full-batch ones, only rows v0..v1-1 of the gradients are written) and ``out=
     (g_fvi, g_ff)`` supplies the full-batch gradient buffers to write into - together they let a
-    caller pipeline view chunks (kaolin_b200.multi_gpu.pipelined_backward_all_gather).
+    caller pipeline view chunks (kaolin_b200.multi_gpu.pipelined_backward_all_gather); being outputs,
+    they are never copied and must be aligned (DIBR_B200_ALIGNMENT).
 
     ``feature_grad_hook`` (per call — there is no process-global state): called as
     ``hook(g_ff)`` between the two branches of a fused backward.  grad_face_features is
     final after the rasterize branch, so e.g. its all-gather can travel while the
     soft-mask branch runs (kaolin_b200.multi_gpu.OverlappedGradAllGather)."""
+    g_feat, g_soft, face_idx, wts, soft, fvi, ff = map(aligned, (g_feat, g_soft, face_idx, wts, soft, fvi, ff))
     dev = fvi.device
     B, F = fvi.shape[0], fvi.shape[1]
     D = 0 if ff is None else ff.shape[-1]
@@ -192,6 +206,7 @@ def backward(height, width, g_feat, g_soft, face_idx, wts, soft, fvi, ff, multip
 def forward_f64(mode, height, width, fvz, fvi, ff, fnz, valid_u8, multiplier, eps, sigmainv, boxlen_m, knum,
                 face_idx_in=None):
     """-> (feat f64, face_idx, weights f64, soft f64, workspace); boxlen_m is a Python float (double)."""
+    fvz, fvi, ff, fnz, valid_u8, face_idx_in = map(aligned, (fvz, fvi, ff, fnz, valid_u8, face_idx_in))
     dev = fvi.device
     B, F = fvi.shape[0], fvi.shape[1]
     D = 0 if ff is None else ff.shape[-1]
@@ -219,6 +234,7 @@ def forward_f64(mode, height, width, fvz, fvi, ff, fnz, valid_u8, multiplier, ep
 
 def backward_f64(height, width, g_feat, g_soft, face_idx, wts, soft, fvi, ff, multiplier, eps, sigmainv, boxlen_m,
                  knum, ws):
+    g_feat, g_soft, face_idx, wts, soft, fvi, ff = map(aligned, (g_feat, g_soft, face_idx, wts, soft, fvi, ff))
     dev = fvi.device
     B, F = fvi.shape[0], fvi.shape[1]
     D = 0 if ff is None else ff.shape[-1]

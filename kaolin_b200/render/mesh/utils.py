@@ -27,13 +27,13 @@ def _proj3(camera_proj):
 class PrepareVerticesB200(Function):
     @staticmethod
     def forward(ctx, vertices, faces, camera_proj, camera_rot, camera_trans, camera_transform):
-        v = vertices.contiguous()
-        f = faces.contiguous()
+        v = _host.aligned(vertices.contiguous())
+        f = _host.aligned(faces.contiguous())
         B, V = v.shape[0], v.shape[1]
         F = f.shape[0]
-        T = None if camera_transform is None else camera_transform.contiguous()
-        R = None if camera_rot is None else camera_rot.contiguous()
-        t = None if camera_trans is None else camera_trans.reshape(B, 3).contiguous()
+        T = None if camera_transform is None else _host.aligned(camera_transform.contiguous())
+        R = None if camera_rot is None else _host.aligned(camera_rot.contiguous())
+        t = None if camera_trans is None else _host.aligned(camera_trans.reshape(B, 3).contiguous())
         proj = _proj3(camera_proj)
         fvc = torch.empty((B, F, 3, 3), dtype=torch.float32, device=v.device)
         fvi = torch.empty((B, F, 3, 2), dtype=torch.float32, device=v.device)
@@ -52,7 +52,7 @@ class PrepareVerticesB200(Function):
         v, f, T, R, t = ctx.saved_tensors
         B, V = v.shape[0], v.shape[1]
         F = f.shape[0]
-        c = lambda g: None if g is None else g.contiguous()
+        c = lambda g: None if g is None else _host.aligned(g.contiguous())
         g_fvc, g_fvi, g_fn = c(g_fvc), c(g_fvi), c(g_fn)
         g_vc = torch.empty((B, V, 3), dtype=torch.float32, device=v.device)
         with torch.cuda.device(v.device):
@@ -115,8 +115,8 @@ def prepare_vertices(vertices, faces, camera_proj, camera_rot=None, camera_trans
 class TextureMappingB200(Function):
     @staticmethod
     def forward(ctx, texture_coordinates, texture_maps, nearest):
-        uv = texture_coordinates.contiguous()
-        tex = texture_maps.contiguous()
+        uv = _host.aligned(texture_coordinates.contiguous())
+        tex = _host.aligned(texture_maps.contiguous())
         B, C, Ht, Wt = tex.shape
         N = uv.numel() // (2 * B)
         out = torch.empty((B, N, C), dtype=torch.float32, device=uv.device)
@@ -138,7 +138,7 @@ class TextureMappingB200(Function):
         g_uv = torch.empty_like(uv) if ctx.needs_input_grad[0] else None
         with torch.cuda.device(uv.device):
             st = _lib.lib().dibr_b200_texture_mapping_backward(
-                B, N, C, Ht, Wt, _host.ptr(uv), _host.ptr(tex), ctx.nearest, _host.ptr(g_out.contiguous()),
+                B, N, C, Ht, Wt, _host.ptr(uv), _host.ptr(tex), ctx.nearest, _host.ptr(_host.aligned(g_out.contiguous())),
                 _host.ptr(g_tex), _host.ptr(g_uv), _host.stream_ptr(uv.device))
         _lib.check(st, "dibr_b200_texture_mapping_backward")
         return g_uv, g_tex, None

@@ -74,6 +74,98 @@ def test_workspace_query_and_host_side_errors():
     assert lib.dibr_b200_peer_push_multicast(ctypes.c_void_p(4096), 32, ctypes.c_void_p(4104), 0, 0, None) == _lib.EINVAL
 
 
+def test_image_size_limit_is_inclusive():
+    """DIBR_B200_MAX_IMAGE_DIM = 16384 px per side is accepted (6 bin levels), 16385 is not."""
+    lib = _lib.lib()
+    for h, w in ((16384, 16384), (16384, 36), (40, 16384)):
+        assert lib.dibr_b200_workspace_bytes(1, 100, h, w) > 0, (h, w)
+        assert lib.dibr_b200_workspace_bytes_f64(1, 100, h, w) > 0, (h, w)
+    for h, w in ((16385, 64), (64, 16385), (16385, 16385)):
+        assert lib.dibr_b200_workspace_bytes(1, 100, h, w) == 0, (h, w)
+        assert lib.dibr_b200_workspace_bytes_f64(1, 100, h, w) == 0, (h, w)
+
+
+def test_misaligned_tensor_pointers_are_rejected_on_the_host():
+    """Every device tensor pointer must be 16-byte aligned (include/dibr_b200.h): the kernels use
+    16-byte vector and cp.async accesses.  A pointer 4 bytes off is refused with EINVAL before any
+    CUDA call.  The calls are built so that, without the alignment check, they would stop at a
+    different host-side result (a too-small workspace, or nothing to do) instead of launching."""
+    lib = _lib.lib()
+    A, M = ctypes.c_void_p(4096), ctypes.c_void_p(4096 + 4)     # aligned / misaligned fake device pointers
+    acc = _lib.ACCUMULATE
+
+    def fwd(fn, **bad):
+        p = {k: A for k in ("fvz", "fvi", "ff", "fnz", "valid", "feat", "idx", "w", "soft")}
+        p.update(bad)
+        return fn(1, 4, 8, 8, 1, p["fvz"], p["fvi"], p["ff"], p["fnz"], p["valid"], 1000.0, 1e-8, 3,
+                  7000.0, 20.0, 30, p["feat"], p["idx"], p["w"], p["soft"], A, 0, None)
+
+    for fn in (lib.dibr_b200_forward, lib.dibr_b200_forward_bf16):
+        assert fwd(fn) == _lib.EWORKSPACE                                # aligned: reaches the workspace check
+        for name in ("fvz", "fvi", "ff", "fnz", "valid", "feat", "idx", "w", "soft"):
+            assert fwd(fn, **{name: M}) == _lib.EINVAL, name
+    assert lib.dibr_b200_forward_f64(1, 4, 8, 8, 1, A, A, A, A, A, 1000.0, 1e-8, 3, 7000.0, 20.0, 30,
+                                     A, A, A, A, A, 0, None) == _lib.EWORKSPACE
+    assert lib.dibr_b200_forward_f64(1, 4, 8, 8, 1, A, M, A, A, A, 1000.0, 1e-8, 3, 7000.0, 20.0, 30,
+                                     A, A, A, A, A, 0, None) == _lib.EINVAL
+
+    # backward, soft-mask branch only, accumulating: the next host check is the workspace size
+    def bwd(fn, **bad):
+        p = {k: A for k in ("gs", "idx", "w", "soft", "fvi", "ff", "gxy", "gff")}
+        p.update(bad)
+        return fn(1, 4, 8, 8, 1, None, p["gs"], p["idx"], p["w"], p["soft"], p["fvi"], p["ff"],
+                  1000.0, 1e-8, 7000.0, 20.0, 30, p["gxy"], p["gff"], A, 0, acc, None)
+
+    for fn in (lib.dibr_b200_backward, lib.dibr_b200_backward_bf16):
+        assert bwd(fn) == _lib.EWORKSPACE
+        for name in ("gs", "idx", "w", "soft", "fvi", "ff", "gxy", "gff"):
+            assert bwd(fn, **{name: M}) == _lib.EINVAL, name
+    # an upstream feature gradient at a 4-byte storage offset (no faces: nothing else to do)
+    for fn in (lib.dibr_b200_backward, lib.dibr_b200_backward_bf16):
+        assert fn(1, 0, 8, 8, 2, M, None, A, A, None, A, A, 1000.0, 1e-8, 7000.0, 20.0, 30,
+                  A, A, None, 0, acc, None) == _lib.EINVAL
+    assert lib.dibr_b200_backward_views(2, 0, 8, 8, 2, M, None, A, A, None, A, A, 1, 1000.0, 1e-8, 7000.0,
+                                        20.0, 30, A, A, None, 0, acc, 1, 2, None) == _lib.EINVAL
+    assert lib.dibr_b200_backward_f64(1, 4, 8, 8, 1, None, M, A, A, A, A, A, 1000.0, 1e-8, 7000.0, 20.0, 30,
+                                      A, A, A, 0, acc, None) == _lib.EINVAL
+    # operators
+    assert lib.dibr_b200_packed_rasterize_forward(1, 4, 8, 8, 1, A, A, M, A, A, 1000.0, 1e-8, A, A, A,
+                                                  A, 0, None) == _lib.EINVAL
+    assert lib.dibr_b200_packed_rasterize_forward(1, 4, 8, 8, 1, A, A, A, A, A, 1000.0, 1e-8, A, A, A,
+                                                  A, 0, None) == _lib.EWORKSPACE
+    assert lib.dibr_b200_rasterize_backward(1, 0, 8, 8, 2, M, A, A, A, A, 1e-8, A, A, None) == _lib.EINVAL
+    assert lib.dibr_b200_soft_mask_forward(1, 4, 8, 8, 30, A, A, A, 7000.0, 1000.0, A, A, M, A,
+                                           A, 0, None) == _lib.EINVAL
+    assert lib.dibr_b200_soft_mask_forward(1, 4, 8, 8, 30, A, A, A, 7000.0, 1000.0, A, A, A, A,
+                                           A, 0, None) == _lib.EWORKSPACE
+    assert lib.dibr_b200_soft_mask_backward(1, 4, 8, 8, 30, A, A, A, A, A, A, M, 7000.0, 1000.0,
+                                            A, None) == _lib.EINVAL
+    assert lib.dibr_b200_deftet_sparse_render_forward(1, 4, 8, 2, A, A, M, A, A, 1e-8, A, A, A, A,
+                                                      A, 0, None) == _lib.EINVAL
+    assert lib.dibr_b200_deftet_sparse_render_forward(1, 4, 8, 2, A, A, A, A, A, 1e-8, A, A, A, A,
+                                                      A, 0, None) == _lib.EWORKSPACE
+    assert lib.dibr_b200_deftet_sparse_render_backward(1, 4, 8, 2, 3, M, A, A, A, A, 1e-8, A, A,
+                                                       None) == _lib.EINVAL
+    assert lib.dibr_b200_texture_mapping_forward(1, 0, 3, 4, 4, M, A, 0, A, None) == _lib.EINVAL
+    assert lib.dibr_b200_texture_mapping_forward(1, 0, 3, 4, 4, A, A, 0, A, None) == 0
+    assert lib.dibr_b200_mask_iou_backward(1, 16, A, A, A, A, M, A, None) == _lib.EINVAL
+
+
+def test_misaligned_views_are_copied_before_the_abi():
+    """The Python layers hand the C ABI a 16-byte aligned copy of a tensor view at a storage offset."""
+    from kaolin_b200.render.mesh import _host
+    buf = torch.zeros(1 + 4 * 3 * 2)
+    t = buf[1:].view(4, 3, 2)
+    assert t.is_contiguous() and t.data_ptr() % 16 == 4
+    c = _host.aligned(t)
+    assert c.data_ptr() % 16 == 0 and torch.equal(c, t) and c.is_contiguous()
+    a = buf[4:].view(-1)
+    assert a.data_ptr() % 16 == 0 and _host.aligned(a) is a            # aligned views are passed through
+    assert _host.aligned(None) is None
+    h = torch.zeros(9, dtype=torch.bfloat16)[1:]
+    assert h.data_ptr() % 16 == 2 and _host.aligned(h).data_ptr() % 16 == 0
+
+
 def test_python_signatures_match_reference():
     """rasterization.py:373-381, dibr.py:75-76,119-122."""
     sig = inspect.signature(rasterize)

@@ -451,7 +451,7 @@ def test_operator_level_vs_oracle():
     assert rel_err(N(gxy), o_gxy) <= GRAD_REL and rel_err(N(gff), o_gff) <= GRAD_REL
 
 
-@pytest.mark.parametrize("D", [1, 2, 5, 9])
+@pytest.mark.parametrize("D", [1, 2, 4, 5, 9])
 def test_feature_dims(D):
     fvz, fvi, fnz = synthetic.icosphere_views(1, 2, seed=8)
     B, F = fvz.shape[:2]
