@@ -260,6 +260,54 @@ int dibr_b200_soft_mask_backward(
     float sigmainv, float multiplier, float* grad_face_vertices_image,
     dibr_b200_stream_t stream);
 
+/*
+ * float64 instantiation of the four operators (the reference dispatches float and double:
+ * rasterization_cuda.cu:218/427, dibr_soft_mask_cuda.cu:205/376).  Each takes the arguments of its
+ * float sibling above, with double tensors where the reference uses scalar_t; indices, K-list ids and
+ * dist types keep their types, multiplier / eps / sigmainv stay C floats as in the reference kernels.
+ * Every decision is the reference's <double> arithmetic on the caller's tensors as given: the half-open
+ * bbox tests read face_bboxes / face_large_bboxes, the coordinates are not multiplied again, pixel
+ * centres are computed in float and widened.  Built for exactness, not speed.  The two forwards take a
+ * workspace of at least dibr_b200_workspace_bytes_f64(); the two backwards zero their outputs inside.
+ */
+
+/* Operator: kaolin::packed_rasterize_forward_cuda<double> (rasterization.h:23-32). */
+int dibr_b200_packed_rasterize_forward_f64(
+    int batch, int64_t total_faces, int height, int width, int feat_dim,
+    const double* face_vertices_z, const double* face_vertices_image,
+    const double* face_bboxes, const double* face_features,
+    const int64_t* first_idx_face_per_mesh, float multiplier, float eps,
+    double* interpolated_features, int64_t* selected_face_idx, double* output_weights,
+    void* workspace, size_t workspace_bytes, dibr_b200_stream_t stream);
+
+/* Operator: kaolin::rasterize_backward_cuda<double> (rasterization.h:34-41); no workspace. */
+int dibr_b200_rasterize_backward_f64(
+    int batch, int num_faces, int height, int width, int feat_dim,
+    const double* grad_interpolated_features, const int64_t* selected_face_idx,
+    const double* output_weights, const double* face_vertices_image,
+    const double* face_features, float eps,
+    double* grad_face_vertices_image, double* grad_face_features,
+    dibr_b200_stream_t stream);
+
+/* Operator: kaolin::dibr_soft_mask_forward_cuda<double> (dibr_soft_mask.h:23-30).  close_face_prob
+ * (B,H,W,K) f64; the three K-lists are all given or all NULL. */
+int dibr_b200_soft_mask_forward_f64(
+    int batch, int num_faces, int height, int width, int knum,
+    const double* face_vertices_image, const double* face_large_bboxes,
+    const int64_t* selected_face_idx, float sigmainv, float multiplier,
+    double* soft_mask, double* close_face_prob, int64_t* close_face_idx,
+    uint8_t* close_face_dist_type,
+    void* workspace, size_t workspace_bytes, dibr_b200_stream_t stream);
+
+/* Operator: kaolin::dibr_soft_mask_backward_cuda<double> (dibr_soft_mask.h:32-42). */
+int dibr_b200_soft_mask_backward_f64(
+    int batch, int num_faces, int height, int width, int knum,
+    const double* grad_soft_mask, const double* soft_mask, const int64_t* selected_face_idx,
+    const double* close_face_prob, const int64_t* close_face_idx,
+    const uint8_t* close_face_dist_type, const double* face_vertices_image,
+    float sigmainv, float multiplier, double* grad_face_vertices_image,
+    dibr_b200_stream_t stream);
+
 /* =========================================================================
  * The steps either side of the rasterizer in every DIB-R caller (SURVEY.md 8f rank 1, 2);
  * kaolin_b200/csrc/mesh_pipeline.cu.  The reference has no native interface for them: they

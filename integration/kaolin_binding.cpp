@@ -21,9 +21,12 @@
 
 namespace {
 
-void check_float(const char* fn, const at::Tensor& t) {
-  TORCH_CHECK(t.scalar_type() == at::kFloat, "\"", fn, "\" not implemented for '", toString(t.scalar_type()),
-              "' (libdibr_b200 computes in float32)");
+// AT_DISPATCH_FLOATING_TYPES: true for double, false for float; any other type is refused in the
+// reference's wording.  The other tensors' data_ptr<scalar_t>() then refuses a mixed float/double call.
+bool is_double(const char* fn, const at::Tensor& t) {
+  TORCH_CHECK(t.scalar_type() == at::kFloat || t.scalar_type() == at::kDouble, "\"", fn, "\" not implemented for '",
+              toString(t.scalar_type()), "'");
+  return t.scalar_type() == at::kDouble;
 }
 
 void check_status(const char* fn, int st) {
@@ -41,8 +44,9 @@ at::Tensor aligned(const at::Tensor& t) {
   return reinterpret_cast<uintptr_t>(t.data_ptr()) % DIBR_B200_ALIGNMENT ? t.clone(at::MemoryFormat::Contiguous) : t;
 }
 
-at::Tensor workspace(const at::Tensor& like, int batch, int64_t faces, int height, int width) {
-  const size_t n = dibr_b200_workspace_bytes(batch, faces, height, width);
+at::Tensor workspace(const at::Tensor& like, int batch, int64_t faces, int height, int width, bool f64 = false) {
+  const size_t n = f64 ? dibr_b200_workspace_bytes_f64(batch, faces, height, width)
+                       : dibr_b200_workspace_bytes(batch, faces, height, width);
   TORCH_CHECK(n > 0, "libdibr_b200: unsupported problem size");
   return at::empty({static_cast<int64_t>(n)}, like.options().dtype(at::kByte));
 }
@@ -69,7 +73,7 @@ std::vector<at::Tensor> packed_rasterize_forward_cuda(
   at::checkSize(__func__, bb_arg, {num_faces, 4});
   at::checkSize(__func__, ff_arg, {num_faces, 3, D});
   at::checkSize(__func__, first_arg, {batch + 1});
-  check_float(__func__, face_vertices_z);
+  const bool f64 = is_double(__func__, face_vertices_z);
   const at::cuda::OptionalCUDAGuard guard(at::device_of(face_vertices_z));
   const at::Tensor z = aligned(face_vertices_z), xy = aligned(face_vertices_image), bb = aligned(face_bboxes),
                    ff = aligned(face_features), first = aligned(first_idx_face_per_mesh);
@@ -77,7 +81,15 @@ std::vector<at::Tensor> packed_rasterize_forward_cuda(
   at::Tensor idx = at::empty({batch, height, width}, opt.dtype(at::kLong));
   at::Tensor w = at::empty({batch, height, width, 3}, opt);
   at::Tensor out = at::empty({batch, height, width, D}, opt);
-  at::Tensor ws = workspace(face_vertices_z, batch, num_faces, height, width);
+  at::Tensor ws = workspace(face_vertices_z, batch, num_faces, height, width, f64);
+  if (f64) {
+    check_status(__func__, dibr_b200_packed_rasterize_forward_f64(
+        batch, num_faces, height, width, D, z.data_ptr<double>(), xy.data_ptr<double>(),
+        bb.data_ptr<double>(), ff.data_ptr<double>(), first.data_ptr<int64_t>(),
+        multiplier, eps, out.data_ptr<double>(), idx.data_ptr<int64_t>(), w.data_ptr<double>(), ws.data_ptr(),
+        static_cast<size_t>(ws.numel()), current_stream()));
+    return {out, idx, w};
+  }
   check_status(__func__, dibr_b200_packed_rasterize_forward(
       batch, num_faces, height, width, D, z.data_ptr<float>(), xy.data_ptr<float>(),
       bb.data_ptr<float>(), ff.data_ptr<float>(), first.data_ptr<int64_t>(),
@@ -107,12 +119,19 @@ std::vector<at::Tensor> rasterize_backward_cuda(
   at::checkSize(__func__, w_arg, {batch, height, width, 3});
   at::checkSize(__func__, xy_arg, {batch, F, 3, 2});
   at::checkSize(__func__, ff_arg, {batch, F, 3, D});
-  check_float(__func__, grad_interpolated_features);
+  const bool f64 = is_double(__func__, grad_interpolated_features);
   const at::cuda::OptionalCUDAGuard guard(at::device_of(grad_interpolated_features));
   const at::Tensor g = aligned(grad_interpolated_features), idx = aligned(selected_face_idx),
                    w = aligned(output_weights), xy = aligned(face_vertices_image), ff = aligned(face_features);
   at::Tensor g_xy = at::empty_like(face_vertices_image);
   at::Tensor g_ff = at::empty_like(face_features);
+  if (f64) {
+    check_status(__func__, dibr_b200_rasterize_backward_f64(
+        batch, F, height, width, D, g.data_ptr<double>(), idx.data_ptr<int64_t>(), w.data_ptr<double>(),
+        xy.data_ptr<double>(), ff.data_ptr<double>(), eps, g_xy.data_ptr<double>(), g_ff.data_ptr<double>(),
+        current_stream()));
+    return {g_xy, g_ff};
+  }
   // the fused entry point with a workspace takes the row-walk scatter kernel
   at::Tensor ws = workspace(face_vertices_image, batch, static_cast<int64_t>(batch) * F, height, width);
   check_status(__func__, dibr_b200_backward(
@@ -139,7 +158,7 @@ std::vector<at::Tensor> dibr_soft_mask_forward_cuda(
   at::checkSize(__func__, xy_arg, {batch, F, 3, 2});
   at::checkSize(__func__, bb_arg, {batch, F, 4});
   at::checkSize(__func__, idx_arg, {batch, height, width});
-  check_float(__func__, face_vertices_image);
+  const bool f64 = is_double(__func__, face_vertices_image);
   const at::cuda::OptionalCUDAGuard guard(at::device_of(face_vertices_image));
   const at::Tensor xy = aligned(face_vertices_image), bb = aligned(face_large_bboxes), idx = aligned(selected_face_idx);
   auto opt = face_vertices_image.options();
@@ -147,7 +166,15 @@ std::vector<at::Tensor> dibr_soft_mask_forward_cuda(
   at::Tensor prob = at::empty({batch, height, width, knum}, opt);
   at::Tensor cidx = at::empty({batch, height, width, knum}, opt.dtype(at::kLong));
   at::Tensor ctype = at::empty({batch, height, width, knum}, opt.dtype(at::kByte));
-  at::Tensor ws = workspace(face_vertices_image, batch, static_cast<int64_t>(batch) * F, height, width);
+  at::Tensor ws = workspace(face_vertices_image, batch, static_cast<int64_t>(batch) * F, height, width, f64);
+  if (f64) {
+    check_status(__func__, dibr_b200_soft_mask_forward_f64(
+        batch, F, height, width, knum, xy.data_ptr<double>(), bb.data_ptr<double>(),
+        idx.data_ptr<int64_t>(), sigmainv, multiplier, soft.data_ptr<double>(), prob.data_ptr<double>(),
+        cidx.data_ptr<int64_t>(), ctype.data_ptr<uint8_t>(), ws.data_ptr(), static_cast<size_t>(ws.numel()),
+        current_stream()));
+    return {soft, prob, cidx, ctype};
+  }
   check_status(__func__, dibr_b200_soft_mask_forward(
       batch, F, height, width, knum, xy.data_ptr<float>(), bb.data_ptr<float>(),
       idx.data_ptr<int64_t>(), sigmainv, multiplier, soft.data_ptr<float>(), prob.data_ptr<float>(),
@@ -179,12 +206,20 @@ at::Tensor dibr_soft_mask_backward_cuda(
   at::checkSize(__func__, ci_arg, {batch, height, width, knum});
   at::checkSize(__func__, ct_arg, {batch, height, width, knum});
   at::checkSize(__func__, xy_arg, {batch, F, 3, 2});
-  check_float(__func__, grad_soft_mask);
+  const bool f64 = is_double(__func__, face_vertices_image);
   const at::cuda::OptionalCUDAGuard guard(at::device_of(grad_soft_mask));
   const at::Tensor g = aligned(grad_soft_mask), soft = aligned(soft_mask), idx = aligned(selected_face_idx),
                    prob = aligned(close_face_prob), cidx = aligned(close_face_idx),
                    ctype = aligned(close_face_dist_type), xy = aligned(face_vertices_image);
   at::Tensor g_xy = at::empty_like(face_vertices_image);
+  if (f64) {
+    check_status(__func__, dibr_b200_soft_mask_backward_f64(
+        batch, F, height, width, knum, g.data_ptr<double>(), soft.data_ptr<double>(),
+        idx.data_ptr<int64_t>(), prob.data_ptr<double>(), cidx.data_ptr<int64_t>(),
+        ctype.data_ptr<uint8_t>(), xy.data_ptr<double>(), sigmainv, multiplier,
+        g_xy.data_ptr<double>(), current_stream()));
+    return g_xy;
+  }
   check_status(__func__, dibr_b200_soft_mask_backward(
       batch, F, height, width, knum, g.data_ptr<float>(), soft.data_ptr<float>(),
       idx.data_ptr<int64_t>(), prob.data_ptr<float>(), cidx.data_ptr<int64_t>(),

@@ -68,6 +68,14 @@ SIGNATURES = {
                                          _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "dibr_b200_soft_mask_backward": (_i, [_i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                           _f, _f, _vp, _vp]),
+    "dibr_b200_packed_rasterize_forward_f64": (_i, [_i, _i64, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f,
+                                                    _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dibr_b200_rasterize_backward_f64": (_i, [_i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f,
+                                              _vp, _vp, _vp]),
+    "dibr_b200_soft_mask_forward_f64": (_i, [_i, _i, _i, _i, _i, _vp, _vp, _vp, _f, _f,
+                                             _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dibr_b200_soft_mask_backward_f64": (_i, [_i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                              _f, _f, _vp, _vp]),
     # SURVEY.md §8(f): the steps either side of the rasterizer (csrc/mesh_pipeline.cu)
     "dibr_b200_prepare_vertices_forward": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, _fp3, _vp, _vp, _vp, _vp]),
     "dibr_b200_prepare_vertices_backward": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, _fp3, _vp, _vp, _vp,

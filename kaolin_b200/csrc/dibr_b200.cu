@@ -2848,6 +2848,134 @@ int dibr_b200_backward_f64(int batch, int num_faces, int height, int width, int 
   return (int)cudaGetLastError();
 }
 
+int dibr_b200_packed_rasterize_forward_f64(int batch, int64_t total_faces, int height, int width, int feat_dim,
+                                           const double* face_vertices_z, const double* face_vertices_image,
+                                           const double* face_bboxes, const double* face_features,
+                                           const int64_t* first_idx_face_per_mesh, float multiplier, float eps,
+                                           double* interpolated_features, int64_t* selected_face_idx,
+                                           double* output_weights, void* workspace, size_t workspace_bytes_,
+                                           dibr_b200_stream_t stream) {
+  int rc = check_dims(batch, total_faces, height, width);
+  if (rc) return rc;
+  if (!selected_face_idx || !output_weights || !first_idx_face_per_mesh || feat_dim < 0 || !(multiplier > 0.f))
+    return DIBR_B200_EINVAL;
+  if (feat_dim > 0 && (!interpolated_features || (total_faces > 0 && !face_features))) return DIBR_B200_EINVAL;
+  if (total_faces > 0 && (!face_vertices_z || !face_vertices_image || !face_bboxes)) return DIBR_B200_EINVAL;
+  if (misaligned(face_vertices_z, face_vertices_image, face_bboxes, face_features, first_idx_face_per_mesh,
+                 interpolated_features, selected_face_idx, output_weights))
+    return DIBR_B200_EINVAL;
+  cudaStream_t st = (cudaStream_t)stream;
+  F64OpArgs a;
+  a.D = feat_dim; a.K = 0; a.eps = eps; a.sigmainv = 0.f; a.multiplier = multiplier;
+  a.xy = face_vertices_image; a.z = face_vertices_z; a.feat = face_features; a.box = face_bboxes;
+  a.out_feat = interpolated_features; a.idx = selected_face_idx; a.out_w = output_weights; a.out_soft = nullptr;
+  a.prob = nullptr; a.cidx = nullptr; a.ctype = nullptr;
+  rc = f64_op_setup(a, batch, total_faces, 0, height, width, first_idx_face_per_mesh, multiplier, 1, workspace,
+                    workspace_bytes_, st);
+  if (rc) return rc;
+  Span sp("f64_raster_op_kernel", st);
+  f64_raster_op_kernel<<<tile_grid(a.s), kThreads, 0, st>>>(a);
+  return (int)cudaGetLastError();
+}
+
+int dibr_b200_rasterize_backward_f64(int batch, int num_faces, int height, int width, int feat_dim,
+                                     const double* grad_interpolated_features, const int64_t* selected_face_idx,
+                                     const double* output_weights, const double* face_vertices_image,
+                                     const double* face_features, float eps, double* grad_face_vertices_image,
+                                     double* grad_face_features, dibr_b200_stream_t stream) {
+  const int64_t NF = (int64_t)batch * num_faces;
+  int rc = check_dims(batch, NF, height, width);
+  if (rc) return rc;
+  if (!selected_face_idx || !grad_face_vertices_image || num_faces < 0 || feat_dim < 0) return DIBR_B200_EINVAL;
+  if (feat_dim > 0 && (!grad_interpolated_features || !output_weights || !grad_face_features ||
+                       (num_faces > 0 && !face_features)))
+    return DIBR_B200_EINVAL;
+  if (num_faces > 0 && !face_vertices_image) return DIBR_B200_EINVAL;
+  if (misaligned(grad_interpolated_features, selected_face_idx, output_weights, face_vertices_image, face_features,
+                 grad_face_vertices_image, grad_face_features))
+    return DIBR_B200_EINVAL;
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(grad_face_vertices_image, 0, (size_t)NF * 6 * sizeof(double), st);
+  if (e != cudaSuccess) return (int)e;
+  if (feat_dim > 0) {
+    e = cudaMemsetAsync(grad_face_features, 0, (size_t)NF * 3 * feat_dim * sizeof(double), st);
+    if (e != cudaSuccess) return (int)e;
+  }
+  if (NF == 0 || feat_dim == 0) return 0;
+  F64Args a = {};
+  a.s.B = batch; a.s.H = height; a.s.W = width; a.s.F = num_faces;
+  a.D = feat_dim; a.eps = eps; a.xy = face_vertices_image; a.feat = face_features;
+  a.idx = const_cast<int64_t*>(selected_face_idx); a.out_w = const_cast<double*>(output_weights);
+  a.g_feat = grad_interpolated_features; a.g_xy = grad_face_vertices_image; a.g_ff = grad_face_features;
+  const int64_t P = (int64_t)batch * height * width;
+  Span sp("f64_raster_bwd_op_kernel", st);
+  f64_raster_bwd_op_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(a);
+  return (int)cudaGetLastError();
+}
+
+int dibr_b200_soft_mask_forward_f64(int batch, int num_faces, int height, int width, int knum,
+                                    const double* face_vertices_image, const double* face_large_bboxes,
+                                    const int64_t* selected_face_idx, float sigmainv, float multiplier,
+                                    double* soft_mask, double* close_face_prob, int64_t* close_face_idx,
+                                    uint8_t* close_face_dist_type, void* workspace, size_t workspace_bytes_,
+                                    dibr_b200_stream_t stream) {
+  const int64_t NF = (int64_t)batch * num_faces;
+  int rc = check_dims(batch, NF, height, width);
+  if (rc) return rc;
+  if (!selected_face_idx || !soft_mask || knum <= 0 || num_faces < 0 || !(multiplier > 0.f)) return DIBR_B200_EINVAL;
+  if (num_faces > 0 && (!face_vertices_image || !face_large_bboxes)) return DIBR_B200_EINVAL;
+  const bool lists = close_face_prob || close_face_idx || close_face_dist_type;
+  if (lists && !(close_face_prob && close_face_idx && close_face_dist_type)) return DIBR_B200_EINVAL;
+  if (lists && (int64_t)batch * height * width * knum < 0) return DIBR_B200_ESIZE;
+  if (misaligned(face_vertices_image, face_large_bboxes, selected_face_idx, soft_mask, close_face_prob,
+                 close_face_idx, close_face_dist_type))
+    return DIBR_B200_EINVAL;
+  cudaStream_t st = (cudaStream_t)stream;
+  F64OpArgs a;
+  a.D = 0; a.K = knum; a.eps = 0.f; a.sigmainv = sigmainv; a.multiplier = multiplier;
+  a.xy = face_vertices_image; a.z = nullptr; a.feat = nullptr; a.box = face_large_bboxes;
+  a.out_feat = nullptr; a.idx = const_cast<int64_t*>(selected_face_idx); a.out_w = nullptr; a.out_soft = soft_mask;
+  a.prob = close_face_prob; a.cidx = close_face_idx; a.ctype = close_face_dist_type;
+  rc = f64_op_setup(a, batch, NF, num_faces, height, width, nullptr, multiplier, 2, workspace, workspace_bytes_, st);
+  if (rc) return rc;
+  Span sp("f64_soft_op_kernel", st);
+  f64_soft_op_kernel<<<tile_grid(a.s), kThreads, 0, st>>>(a);
+  return (int)cudaGetLastError();
+}
+
+int dibr_b200_soft_mask_backward_f64(int batch, int num_faces, int height, int width, int knum,
+                                     const double* grad_soft_mask, const double* soft_mask,
+                                     const int64_t* selected_face_idx, const double* close_face_prob,
+                                     const int64_t* close_face_idx, const uint8_t* close_face_dist_type,
+                                     const double* face_vertices_image, float sigmainv, float multiplier,
+                                     double* grad_face_vertices_image, dibr_b200_stream_t stream) {
+  const int64_t NF = (int64_t)batch * num_faces;
+  int rc = check_dims(batch, NF, height, width);
+  if (rc) return rc;
+  if (!grad_soft_mask || !soft_mask || !selected_face_idx || !close_face_prob || !close_face_idx ||
+      !close_face_dist_type || !grad_face_vertices_image || knum <= 0 || num_faces < 0 || !(multiplier > 0.f))
+    return DIBR_B200_EINVAL;
+  if (num_faces > 0 && !face_vertices_image) return DIBR_B200_EINVAL;
+  if (misaligned(grad_soft_mask, soft_mask, selected_face_idx, close_face_prob, close_face_idx,
+                 close_face_dist_type, face_vertices_image, grad_face_vertices_image))
+    return DIBR_B200_EINVAL;
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(grad_face_vertices_image, 0, (size_t)NF * 6 * sizeof(double), st);
+  if (e != cudaSuccess) return (int)e;
+  if (NF == 0) return 0;
+  F64SoftBwdArgs a;
+  a.B = batch; a.H = height; a.W = width; a.F = num_faces; a.K = knum;
+  a.grid = make_grid(multiplier, width, height);
+  a.sigmainv = sigmainv; a.multiplier = multiplier;
+  a.grad_soft = grad_soft_mask; a.soft = soft_mask; a.idx = selected_face_idx;
+  a.prob = close_face_prob; a.cidx = close_face_idx; a.ctype = close_face_dist_type;
+  a.xy = face_vertices_image; a.grad_xy = grad_face_vertices_image;
+  const int64_t P = (int64_t)batch * height * width;
+  Span sp("f64_soft_bwd_op_kernel", st);
+  f64_soft_bwd_op_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(a);
+  return (int)cudaGetLastError();
+}
+
 int dibr_b200_trace_begin(void) {
   g_trace.on = true;
   g_trace.used = 0;
